@@ -2,7 +2,7 @@
 """bench.py -- frames/s of the nnnoiseless per-frame denoise path on B200 (driver contract).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
-                    [--streams B_per_gpu | --total-streams B] [--frames T] [--model PATH]
+                    [--streams B_per_gpu | --total-streams B] [--frames T] [--model PATH] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch: B streams per GPU, each advanced T consecutive
 480-sample frames (T frame-steps of 5 kernels each, T = 100 = one second of audio per stream, SURVEY 8(d)).
@@ -18,6 +18,9 @@ T*B*1920 B of input (12.6 GB at the default, >> the 126 MB L2).
 --impl reference times the reference's CPU implementation of the same path (the C restatement in
 oracle/ -- the Rust crate cannot be built in this image) with all host threads, pinned, on a bounded sample of
 the same workload.
+
+--dump-outputs DIR writes what the last timed step returned (see dump_outputs).  The inputs are seeded and the warm-up
+steps start from a fresh state, so two builds run with the same arguments can be compared output for output.
 """
 import os
 
@@ -353,6 +356,25 @@ def run_reference(args):
     print(json.dumps(line))
 
 
+DUMP_BYTES = 64_000_000  # --dump-outputs writes at most this much in all
+
+
+def dump_outputs(torch, path, out, vad):
+    """--dump-outputs: what the last timed step returned, as float32 .npy files under `path`.  vad.npy is the [T][B]
+    voice probability, whole when it takes at most half of DUMP_BYTES; out.npy is the denoised [n][480] frames of the
+    (frame, stream) pairs in a fixed sample (seed 0, in row-major [T][B] order) that fills the other half, or of every
+    pair when they fit.  vad.npy is sampled at the same pairs when it is not whole."""
+    T, B = vad.shape
+    rows = T * B
+    n = min(rows, DUMP_BYTES // 2 // (FRAME * 4))
+    idx = np.arange(rows) if n == rows else np.sort(np.random.default_rng(0).choice(rows, n, replace=False))
+    idx_d = torch.from_numpy(idx).to(out.device)
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "out.npy"), out.reshape(rows, FRAME).index_select(0, idx_d).cpu().numpy())
+    v = vad if rows * 4 <= DUMP_BYTES // 2 else vad.reshape(rows).index_select(0, idx_d)
+    np.save(os.path.join(path, "vad.npy"), v.cpu().numpy())
+
+
 def run_b200(args):
     cpus0 = all_cpus()
     # stdout carries exactly ONE JSON line: whatever libraries print on the way (e.g. the NCCL version banner, written by
@@ -432,15 +454,17 @@ def run_b200(args):
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
-    for _ in range(args.warmup):
-        step()
-    barrier()
-    if rank == 0:
         # nvidia-smi needs a moment to start: keep the GPU under the same load until the first sample has arrived
         t_wait = time.time()
         while sampler.proc is not None and os.path.getsize(sampler.path) == 0 and time.time() - t_wait < 5.0:
             step()
             torch.cuda.synchronize()
+    barrier()
+    # exactly `warmup` steps from a fresh state precede the timed ones: what the last timed step computes depends on the
+    # arguments alone, not on how many steps the wait above took
+    batch.reset()
+    for _ in range(args.warmup):
+        step()
     barrier()
     l0 = nb.kernel_launches()
     ps0 = batch.pitch_stats()
@@ -454,6 +478,8 @@ def run_b200(args):
     launches = nb.kernel_launches() - l0
     ps1 = batch.pitch_stats()
     clocks = sampler.stop() if rank == 0 else None
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(torch, args.dump_outputs, out, vad)
     if world > 1:
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
     ms_total = float(ms.item())
@@ -619,7 +645,11 @@ def main():
     ap.add_argument("--e2e-frames", type=int, default=0, help="frames per host-API call in the e2e leg (0 = min(frames, 16))")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-legacy", action="store_true")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write what the last timed step returned (rank 0) as DIR/out.npy and DIR/vad.npy, at most 64 MB")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":

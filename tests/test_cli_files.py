@@ -1,7 +1,7 @@
 """SURVEY §8(f) N2: the file front-end of the reference's `nnnoiseless` binary (src/nnnoiseless.rs; tests/cli.rs).
 
-CPU: decoders against an independent restatement (and against the reference's own fixtures when the reference tree is
-mounted), the WAV writer against Python's `wave`, the CLI's error behaviour, the oracle resampler's properties.
+CPU: decoders against an independent restatement (also on excerpts of the reference's own WAV fixtures), the WAV writer
+against Python's `wave`, the CLI's error behaviour, the oracle resampler's properties.
 GPU: resampler and whole-file results against the oracle."""
 import os
 import struct
@@ -15,7 +15,7 @@ import oracle
 from nnnoiseless_b200 import files
 from nnnoiseless_b200.synth import synth_streams
 
-REF_DATA = "/root/reference/test_data"
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
 def _wav_bytes(x, rate, bits=16, fmt=1, extensible=False, extra_chunk=False):
@@ -64,13 +64,14 @@ def test_wav_decoder_matches_restatement(tmp_path, kw):
         assert np.array_equal(got, np.round(x))                           # >= 16 bits: lossless round trip
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_DATA), reason="reference tree not mounted (GPU box)")
 @pytest.mark.parametrize("name,ch", [("mono.wav", 1), ("stereo.wav", 2), ("mono-float.wav", 1)])
 def test_reference_fixtures_decode(name, ch):
-    path = os.path.join(REF_DATA, name)
+    """The reference's test_data/<name> (written by hound) cut to frames 60000..64095: every chunk before `data` kept
+    byte for byte (mono-float.wav's `fact` and `PEAK` included), the RIFF and data sizes set to the excerpt's."""
+    path = os.path.join(GOLDEN, name.replace(".wav", "_excerpt.wav"))
     got, rate = files.read_audio(path)
     want, wrate = oracle.decode_wav(open(path, "rb").read())
-    assert rate == wrate == 44100.0 and got.shape[1] == ch
+    assert rate == wrate == 44100.0 and got.shape == (4096, ch)
     assert np.array_equal(got, want)
 
 

@@ -3,9 +3,10 @@ include/rnnoise.h declares, parses models exactly like the reference, and refuse
 import ctypes as C
 import os
 import re
+import subprocess
+import sys
 
 import numpy as np
-import pytest
 
 import nnnoiseless_b200 as nb
 import oracle
@@ -87,13 +88,17 @@ def test_model_from_file_takes_over_file(tmp_path, builtin_bytes):
 
 
 def test_no_cpu_fallback():
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
-    with pytest.raises(nb.NnnoiselessError, match="no CUDA device"):
-        nb.DenoiseBatch(4)
-    with pytest.raises(nb.NnnoiselessError):
-        nb.DenoiseState()
+    """Without a visible CUDA device the constructors raise; a child process with every GPU hidden checks this on a
+    machine that has one too."""
+    code = ("import pytest\n"
+            "import nnnoiseless_b200 as nb\n"
+            "with pytest.raises(nb.NnnoiselessError, match='no CUDA device'):\n"
+            "    nb.DenoiseBatch(4)\n"
+            "with pytest.raises(nb.NnnoiselessError):\n"
+            "    nb.DenoiseState()\n")
+    r = subprocess.run([sys.executable, "-c", code], cwd=ROOT, env=dict(os.environ, CUDA_VISIBLE_DEVICES=""),
+                       capture_output=True, text=True, timeout=300)
+    assert r.returncode == 0, r.stdout + r.stderr
 
 
 def test_product_never_imports_oracle():
