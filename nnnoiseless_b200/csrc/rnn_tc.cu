@@ -216,8 +216,18 @@ __global__ void __launch_bounds__(NT, 1) rnn_tc_kernel(BatchBuffers bb, DeviceMo
     asm volatile("tcgen05.fence::after_thread_sync;\n" ::: "memory");
     const uint32_t tmem = *tmem_slot;
     Row R{tmem + ((uint32_t)(32 * q) << 16), ch};
+    {
+        // the A operand starts as zeros: a K chunk may span columns that no epilogue writes (the padding before the
+        // r * h segment, its tail beyond this layer's width), where the weights are 0 -- but fresh TMEM holds anything,
+        // and 0 * NaN is NaN
+        const float zero8[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+        for (int g = ch; g < A_MAX_HALVES / 8; g += NCH) R.put_act(8 * g, zero8);
+    }
+    asm volatile("tcgen05.wait::st.sync.aligned;\n" ::: "memory");
+    asm volatile("tcgen05.fence::before_thread_sync;\n" ::: "memory");
+    __syncthreads();
+    asm volatile("tcgen05.fence::after_thread_sync;\n" ::: "memory");
     mbar_wait(&bars[1], 0);  // weights, biases and the tanh table have landed
-
     uint32_t par = 0;  // parity of bars[0]
     const int SS = m.state_size;
     const int so_n = m.nv, so_d = m.nv + m.nn;  // state offsets in HBM (vad | noise | denoise)
@@ -425,10 +435,16 @@ __global__ void __launch_bounds__(NT, 1) rnn_tc_kernel(BatchBuffers bb, DeviceMo
 
 inline int pad8(int n) { return (n + 7) & ~7; }
 inline int pad16(int n) { return (n + 15) & ~15; }
+// dynamic shared memory of rnn_tc_kernel: model image, the feature operand at the next 1 KB boundary, two mbarriers and
+// the TMEM address (the layout at the top of the kernel)
+inline size_t tc_smem_bytes(const DeviceModelTc& d) {
+    return (((size_t)d.blob_bytes + 1023) & ~(size_t)1023) + 2 * 2 * FEAT_CHUNKS * FEAT_GROUP_BYTES + 64;
+}
 
 }  // namespace
 
-// ---- host: pack the model for the kernel.  Returns false if the model does not fit the TMEM / shared-memory budget. ----
+// ---- host: pack the model image for the kernel (weights, biases, tanh table).  Returns false if the model does not fit
+// the TMEM / shared-memory budget. ----
 bool build_model_tc(const HostModel& hm, DeviceModelTc* d, std::vector<unsigned char>* blob) {
     const int nd = hm.input_dense.nn, nv = hm.vad_gru.nn, nn = hm.noise_gru.nn, ndn = hm.denoise_gru.nn;
     d->nd = nd; d->nv = nv; d->nn = nn; d->ndn = ndn;
@@ -475,10 +491,17 @@ bool build_model_tc(const HostModel& hm, DeviceModelTc* d, std::vector<unsigned 
         std::vector<int> entries(chunks.begin(), chunks.end());
         if (use_feat)
             for (int f = 0; f < FEAT_CHUNKS; f++) entries.push_back(-(f + 1));
+        const int np = ngates * p8;
+        if (np == 0) {
+            entries.clear();  // a zero-width layer has no accumulators: issue no MMA (N = 0 is not an MMA shape)
+        } else if (entries.empty()) {
+            // accumulators that are read but that no input feeds (a zero-width input layer): one zero-weight chunk of
+            // the feature operand, which always holds finite values, makes them 0 instead of leaving stale TMEM
+            entries.push_back(-1);
+        }
         if ((int)entries.size() > 16) return false;
         ph.nk = (int)entries.size();
         for (int i = 0; i < ph.nk; i++) ph.chunk[i] = (short)entries[i];
-        const int np = ngates * p8;
         ph.n = pad16(np);
         if (ph.n > 256 || d_col + ph.n > D_COLS) return false;
         ph.d_col = d_col;
@@ -498,7 +521,7 @@ bool build_model_tc(const HostModel& hm, DeviceModelTc* d, std::vector<unsigned 
                         if (w.seg == seg && j < w.len) src = B + (w.recurrent ? r_off : w_off) + (size_t)(w.row0 + j) * row_stride;
                 } else {
                     const int j = (-entries[kc] - 1) * 16 + kk;
-                    if (j < NB_FEATURES) src = B + w_off + (size_t)(feat_row0 + j) * row_stride;
+                    if (use_feat && j < NB_FEATURES) src = B + w_off + (size_t)(feat_row0 + j) * row_stride;
                 }
                 const int k = kc * 16 + kk;
                 for (int n = 0; n < ph.n; n++) {
@@ -531,11 +554,12 @@ bool build_model_tc(const HostModel& hm, DeviceModelTc* d, std::vector<unsigned 
     ok = ok && add_phase(PH_VAD_H, {{0, nd, 0, false}, {4, nv, 0, true}}, false, 0, nv, 1, 2, d->p_v, G1.w_off, G1.r_off, G1.b_off, 3 * nv, 2 * d->p_v > 64 ? 2 * d->p_v : 64);
     // vad_output: one neuron from the vad state; accumulators at the top of the D region
     ok = ok && add_phase(PH_VAD_OUT, {{1, nv, 0, false}}, false, 0, 1, 1, 0, 8, LV.w_off, 0, LV.b_off, 1, D_COLS - 16);
-    // noise_gru: input = [dense_out | vad_state | features]
+    // noise_gru: input = [dense_out | vad_state | features]; the candidate's accumulators reuse the reset gate's columns
+    // (the z | r epilogue has moved r into the A operand before the candidate phase is issued)
     ok = ok && add_phase(PH_NOISE_ZR, {{0, nd, 0, false}, {1, nv, nd, false}, {2, nn, 0, true}}, true, nd + nv, nn, 2, 0, d->p_n, G2.w_off, G2.r_off,
                          G2.b_off, 3 * nn, 0);
     ok = ok && add_phase(PH_NOISE_H, {{0, nd, 0, false}, {1, nv, nd, false}, {4, nn, 0, true}}, true, nd + nv, nn, 1, 2, d->p_n, G2.w_off, G2.r_off,
-                         G2.b_off, 3 * nn, 2 * d->p_n);
+                         G2.b_off, 3 * nn, d->p_n);
     // denoise_gru: input = [vad_state | noise_state | features]; the candidate's accumulators reuse the reset gate's columns
     ok = ok && add_phase(PH_DEN_ZR, {{1, nv, 0, false}, {2, nn, nv, false}, {3, ndn, 0, true}}, true, nv + nn, ndn, 2, 0, d->p_dn, G3.w_off, G3.r_off,
                          G3.b_off, 3 * ndn, 0);
@@ -544,25 +568,25 @@ bool build_model_tc(const HostModel& hm, DeviceModelTc* d, std::vector<unsigned 
     // denoise_output
     ok = ok && add_phase(PH_OUT, {{3, ndn, 0, false}}, false, 0, NB_BANDS, 1, 0, pad8(NB_BANDS), LO.w_off, 0, LO.b_off, NB_BANDS, 0);
     if (!ok) return false;
-    // the noise GRU's candidate must not overlap vad_output's accumulators, which are read after the noise z|r epilogue
-    if (d->ph[PH_NOISE_ZR].n > D_COLS - 16 || d->ph[PH_NOISE_H].d_col + d->ph[PH_NOISE_H].n > D_COLS) return false;
+    // neither noise GRU phase may overlap vad_output's accumulators (columns D_COLS - 16 ..), which are read after the
+    // noise GRU's candidate phase
+    if (d->ph[PH_NOISE_ZR].n > D_COLS - 16 || d->ph[PH_NOISE_H].d_col + d->ph[PH_NOISE_H].n > D_COLS - 16) return false;
     (void)seg_size;
-    return true;
+    // the tanh table closes the image; image + feature operand + barriers must fit one CTA's shared memory
+    while (blob->size() % 16) blob->push_back(0);
+    d->table_off = (uint32_t)blob->size();
+    blob->resize(blob->size() + 208 * 4, 0);
+    std::memcpy(blob->data() + d->table_off, kTansigTable, 201 * 4);
+    while (blob->size() % 16) blob->push_back(0);
+    d->blob_bytes = (uint32_t)blob->size();
+    return tc_smem_bytes(*d) <= 227 * 1024;
 }
 
 int upload_model_tc(const HostModel& hm, UploadedTc* u, cudaStream_t st) {
     u->ok = false;
     std::vector<unsigned char> blob;
     if (!build_model_tc(hm, &u->dm, &blob)) return 0;  // not an error: the caller uses the mma.sync kernel
-    while (blob.size() % 16) blob.push_back(0);
-    u->dm.table_off = (uint32_t)blob.size();
-    blob.resize(blob.size() + 208 * 4, 0);
-    std::memcpy(blob.data() + u->dm.table_off, kTansigTable, 201 * 4);
-    while (blob.size() % 16) blob.push_back(0);
-    u->dm.blob_bytes = (uint32_t)blob.size();
-    const size_t feat_off = (blob.size() + 1023) & ~(size_t)1023;
-    u->smem_bytes = feat_off + 2 * 2 * FEAT_CHUNKS * FEAT_GROUP_BYTES + 64;
-    if (u->smem_bytes > 227 * 1024) return 0;
+    u->smem_bytes = tc_smem_bytes(u->dm);
     if (cudaMalloc(&u->d_blob, blob.size()) != cudaSuccess) return -1;
     if (cudaMemcpyAsync(u->d_blob, blob.data(), blob.size(), cudaMemcpyHostToDevice, st) != cudaSuccess) return -1;
     if (cudaStreamSynchronize(st) != cudaSuccess) return -1;
@@ -607,7 +631,10 @@ void free_model_tc(UploadedTc* u) {
 
 // ---- host-side self test of the PACKING (no GPU): replays the kernel's phase structure in plain f32 from the packed
 // blob and compares with a direct evaluation of src/rnn.rs:343-379 from the model bytes.  Returns the largest absolute
-// difference over gains, vad and the new GRU states (-1: model rejected, -2: model does not fit the tcgen05 budget). ----
+// difference over gains, vad and the new GRU states (+inf if any is NaN); -1: model rejected, -2: model does not fit the
+// tcgen05 budget of TMEM columns or shared memory (the mma.sync kernel runs it), -3: a phase whose accumulators the
+// kernel reads has no K chunk (no MMA would write them), or a phase without accumulators has one (an MMA with N = 0).  Like TMEM, the replay's accumulators start as NaN and a phase only
+// writes its own columns, so an epilogue that reads columns another phase has overwritten, or that no phase wrote, shows. ----
 namespace nnb {
 namespace {
 float h_tansig(float x) {
@@ -631,6 +658,8 @@ extern "C" double nnb_tc_pack_selftest(const unsigned char* bytes, size_t len, i
     DeviceModelTc d{};
     std::vector<unsigned char> blob;
     if (!build_model_tc(hm, &d, &blob)) return -2.0;
+    for (int p = 0; p < TC_PHASES; p++)
+        if ((d.ph[p].n > 0) != (d.ph[p].nk > 0)) return -3.0;
     const int8_t* B = hm.bytes.data();
     const int nd = d.nd, nv = d.nv, nn = d.nn, ndn = d.ndn;
     srand(seed);
@@ -684,7 +713,9 @@ extern "C" double nnb_tc_pack_selftest(const unsigned char* bytes, size_t len, i
     std::vector<float> rg = dense(hm.denoise_output, rd);
 
     // ---- replay of the kernel's phases from the blob ----
-    std::vector<float> A(A_MAX_HALVES + 16, 0.0f), F(16 * FEAT_CHUNKS, 0.0f), D(D_COLS, 0.0f);
+    // the kernel zeroes its A operand once; a chunk past it would read other TMEM columns
+    std::vector<float> A(A_MAX_HALVES + 16, 0.0f), F(16 * FEAT_CHUNKS, 0.0f), D(D_COLS, std::nanf(""));
+    for (int j = A_MAX_HALVES; j < A_MAX_HALVES + 16; j++) A[j] = std::nanf("");
     for (int j = 0; j < NB_FEATURES; j++) F[j] = feat[j];
     for (int j = 0; j < nv; j++) A[d.o_vad + j] = sv[j];
     for (int j = 0; j < nn; j++) A[d.o_noise + j] = sn[j];
@@ -692,6 +723,7 @@ extern "C" double nnb_tc_pack_selftest(const unsigned char* bytes, size_t len, i
     auto run = [&](int p) {
         const TcPhase& ph = d.ph[p];
         const __half* wb = reinterpret_cast<const __half*>(blob.data() + ph.w_off);
+        if (ph.nk == 0) return;  // no MMA is issued: the columns keep what they held
         for (int n = 0; n < ph.n; n++) {
             float acc = 0.0f;
             for (int kc = 0; kc < ph.nk; kc++)
@@ -733,10 +765,15 @@ extern "C" double nnb_tc_pack_selftest(const unsigned char* bytes, size_t len, i
     evad = h_act(d.act_vadout, (D[d.ph[PH_VAD_OUT].d_col] + bias(PH_VAD_OUT)[0]) / 256.0f);
     gru(PH_DEN_ZR, PH_DEN_H, -1, d.act_den, ndn, d.p_dn, ed, d.o_den);
     run(PH_OUT);
-    double worst = std::fabs(evad - rvad);
-    for (int o = 0; o < NB_BANDS; o++) worst = std::max(worst, (double)std::fabs(h_act(d.act_out, (D[d.ph[PH_OUT].d_col + o] + bias(PH_OUT)[o]) / 256.0f) - rg[o]));
-    for (int o = 0; o < nv; o++) worst = std::max(worst, (double)std::fabs(ev[o] - rv[o]));
-    for (int o = 0; o < nn; o++) worst = std::max(worst, (double)std::fabs(en[o] - rn[o]));
-    for (int o = 0; o < ndn; o++) worst = std::max(worst, (double)std::fabs(ed[o] - rd[o]));
+    double worst = 0.0;
+    auto diff = [&](float a, float b) {
+        const double e = std::fabs((double)a - (double)b);
+        worst = std::isnan(e) ? INFINITY : std::max(worst, e);
+    };
+    diff(evad, rvad);
+    for (int o = 0; o < NB_BANDS; o++) diff(h_act(d.act_out, (D[d.ph[PH_OUT].d_col + o] + bias(PH_OUT)[o]) / 256.0f), rg[o]);
+    for (int o = 0; o < nv; o++) diff(ev[o], rv[o]);
+    for (int o = 0; o < nn; o++) diff(en[o], rn[o]);
+    for (int o = 0; o < ndn; o++) diff(ed[o], rd[o]);
     return worst;
 }

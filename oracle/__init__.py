@@ -88,6 +88,7 @@ def lib():
         L.nno_tansig.argtypes = [C.c_float]
         L.nno_sigmoid.restype = C.c_float
         L.nno_sigmoid.argtypes = [C.c_float]
+        L.nno_tansig_table.restype = C.POINTER(C.c_float)
         L.nno_run_batch.restype = C.c_double
         L.nno_run_batch.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                     C.c_int, C.c_int, C.c_int, C.POINTER(C.c_int)]
@@ -159,6 +160,11 @@ class State:
         if getattr(self, "_h", None):
             lib().nno_state_free(self._h)
             self._h = None
+
+
+def tansig_table() -> np.ndarray:
+    """The 201-entry table of the reference's table tanh (src/util.rs:3-27), float32 values, entry i at x = i / 25."""
+    return np.ctypeslib.as_array(lib().nno_tansig_table(), shape=(201,)).copy()
 
 
 def set_fft_mode(mode: int):

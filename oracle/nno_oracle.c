@@ -304,6 +304,7 @@ float nno_tansig(float x) {
     y = y + x * dy * (1.0f - y * x);
     return sign * y;
 }
+const float *nno_tansig_table(void) { return TANSIG_TABLE; }
 /* src/util.rs:47-49 */
 float nno_sigmoid(float x) { return 0.5f + 0.5f * nno_tansig(0.5f * x); }
 /* src/util.rs:51-53 */

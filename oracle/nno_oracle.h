@@ -70,6 +70,8 @@ int32_t nno_pitch_only(nno_state *s, const float *buf1728);
 void nno_set_fft_mode(int mode);
 float nno_tansig(float x);
 float nno_sigmoid(float x);
+/* the 201-entry table behind nno_tansig (src/util.rs:3-27) */
+const float *nno_tansig_table(void);
 
 /*
  * Batched driver used as the timed CPU baseline: n_streams independent states,
